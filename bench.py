@@ -127,6 +127,26 @@ def traversal_bytes(rays, box, prim):
     return 48.0 * rays + 32.0 * box + 48.0 * prim
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def write_outputs(out_dir, frame):
+    """--dump-outputs: the frame of the last timed step as out_dir/image.npy ([H, W, 3], float32 or float64 as rendered), so
+    that two builds can be compared output for output. A frame over 64 MB is replaced by a fixed, seeded sample of its pixels:
+    image_sample.npy [n, 3] and their flat pixel indices, image_sample_index.npy (float64)."""
+    os.makedirs(out_dir, exist_ok=True)
+    frame = np.ascontiguousarray(frame)
+    assert frame.dtype in (np.float32, np.float64), frame.dtype
+    if frame.nbytes <= DUMP_LIMIT_BYTES:
+        np.save(os.path.join(out_dir, "image.npy"), frame)
+        return
+    pixels = frame.reshape(-1, 3)
+    n = DUMP_LIMIT_BYTES // (3 * pixels.itemsize + 8)
+    idx = np.sort(np.random.default_rng(0).choice(len(pixels), n, replace=False))
+    np.save(os.path.join(out_dir, "image_sample.npy"), pixels[idx])
+    np.save(os.path.join(out_dir, "image_sample_index.npy"), idx.astype(np.float64))
+
+
 # ------------------------------------------------------------------------------------- reference arm
 def reference_sample(workload, seconds_target, threads=-1):
     """The unmodified reference on a bounded sample of the workload: the SAME frame (scene, camera,
@@ -171,8 +191,10 @@ def run_reference_arm(args):
         s.render(threads=cores)
     tot_rays, tot_sec = 0, 0.0
     for _ in range(args.steps):
-        _, sec, rays, _ = s.render(threads=cores)
+        img, sec, rays, _ = s.render(threads=cores)
         tot_rays += rays; tot_sec += sec
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, img)
     value = tot_rays / tot_sec / 1e6
     sample = (f"full {s.width}x{s.height} frame at {k * k} spp instead of {WORKLOADS[args.workload][2]['sqrtspp'] ** 2} "
               f"({tot_rays // max(1, args.steps)} rays/step), unmodified reference, best of {{hw, hw/2, ...}} = {cores} threads")
@@ -290,8 +312,9 @@ def parse_ncu_output(text):
     return out
 
 
-def measure(env, args, workload, steps, warmup, sqrtspp_override=0, profile=True):
-    """Times `steps` renders of `workload` on this job's GPUs. -> result dict on rank 0 (None elsewhere)."""
+def measure(env, args, workload, steps, warmup, sqrtspp_override=0, profile=True, dump_dir=None):
+    """Times `steps` renders of `workload` on this job's GPUs; with `dump_dir`, rank 0 writes the frame of the last timed
+    step there (write_outputs). -> result dict on rank 0 (None elsewhere)."""
     torch, dist, m, mdist = env["torch"], env["dist"], env["m"], env["mdist"]
     rank, local_rank, world = env["rank"], env["local_rank"], env["world"]
     pack, _, ov, label = WORKLOADS[workload]
@@ -347,10 +370,12 @@ def measure(env, args, workload, steps, warmup, sqrtspp_override=0, profile=True
     sync_all()
     wall = time.perf_counter() - wall0
     clocks = sampler.stop()
+    # copied before the e2e leg, which renders into the same frames when N > 1
+    last_frame = frames.tensor().cpu().numpy() if dump_dir and rank == 0 else None
 
     # ---- e2e: host buffers in, host buffers out. N=1: the plain C-ABI call mcrt_scene_upload + mcrt_render_rows
     # (float64 frame to the host). N>1: scene upload + sharded render + rank 0 reads the assembled float3 frame.
-    e2e_steps = max(1, min(steps, 3))
+    e2e_steps = steps
     host64 = torch.empty((H, W, 3), dtype=torch.float64).pin_memory() if world == 1 else None
     host32 = torch.empty((H, W, 3), dtype=torch.float32).pin_memory() if world > 1 else None
     frame_t = frames.tensor() if world > 1 else None
@@ -415,6 +440,8 @@ def measure(env, args, workload, steps, warmup, sqrtspp_override=0, profile=True
 
     if rank != 0:
         return None
+    if last_frame is not None:
+        write_outputs(dump_dir, last_frame)
     peak, peak_src = measured_peaks()
     alg_bytes = traversal_bytes(ext_rays, ext_box, ext_prim)
     achieved = alg_bytes / (ext_ms * 1e-3) / 1e9 if ext_ms > 0 else 0.0
@@ -496,12 +523,12 @@ def run_gpu_arm(args):
            "m": importlib.import_module("monte-carlo-ray-tracer_b200"),
            "mdist": importlib.import_module("monte-carlo-ray-tracer_b200.distributed")}
 
-    line = measure(env, args, args.workload, args.steps, args.warmup, args.sqrtspp, profile=not args.no_profile)
+    line = measure(env, args, args.workload, args.steps, args.warmup, args.sqrtspp, profile=not args.no_profile, dump_dir=args.dump_outputs)
     # secondary block: the 457 k-triangle spaceship (BASELINE config 3) at a sample count that keeps the default run short
     secondary = None
     sec_pack = os.path.join(ROOT, WORKLOADS["c3"][0])
     if args.workload == "c2" and not args.no_secondary and not args.sqrtspp and os.path.exists(sec_pack):
-        secondary = measure(env, args, "c3", 3, 3, 8, profile=not args.no_profile)
+        secondary = measure(env, args, "c3", args.steps, args.warmup, 8, profile=not args.no_profile)
 
     if rank == 0:
         if secondary is not None:
@@ -544,7 +571,11 @@ def main():
     ap.add_argument("--no-e2e", action="store_true", help="skip the host-buffer end-to-end leg (long single-purpose runs only)")
     ap.add_argument("--child-render", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--baseline-seconds", type=float, default=0.0, help="reference arm: target seconds per step")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the frame of the last timed step to DIR/image.npy (inputs are fixed: same arguments, same frame)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and not args.sqrtspp and args.workload == "c2":   # the contract's W >= 3 for the headline workload
         args.warmup = 3
     if args.child_render:

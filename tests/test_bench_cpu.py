@@ -27,13 +27,38 @@ def test_reference_arm_json_contract():
     assert "workload" in line["config"]
 
 
-def test_ncu_epilogue_parser():
-    """bench.py's non-timed ncu epilogue: per-kernel DRAM bytes / FP64 instructions / lanes from `ncu --csv` rows and the
-    child's counters (a synthetic capture; the real one runs on the GPU box)."""
+def load_bench():
     import importlib.util
     spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
     bench = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(bench)
+    return bench
+
+
+def test_dump_outputs_writer(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: the frame as image.npy; over the size limit, the same seeded pixel sample every time."""
+    import numpy as np
+    bench = load_bench()
+    frame = np.random.default_rng(1).random((6, 8, 3), dtype=np.float32)
+    bench.write_outputs(str(tmp_path / "full"), frame)
+    assert np.array_equal(np.load(tmp_path / "full" / "image.npy"), frame)
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 400)
+    for run in ("a", "b"):
+        bench.write_outputs(str(tmp_path / run), frame)
+    a = {n: np.load(tmp_path / "a" / (n + ".npy")) for n in ("image_sample", "image_sample_index")}
+    assert sum(v.nbytes for v in a.values()) <= 400 and a["image_sample_index"].dtype == np.float64
+    assert np.array_equal(a["image_sample"], frame.reshape(-1, 3)[a["image_sample_index"].astype(int)])
+    for n, v in a.items():
+        assert np.array_equal(np.load(tmp_path / "b" / (n + ".npy")), v)
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "0"])
+    with pytest.raises(SystemExit):
+        bench.main()
+
+
+def test_ncu_epilogue_parser():
+    """bench.py's non-timed ncu epilogue: per-kernel DRAM bytes / FP64 instructions / lanes from `ncu --csv` rows and the
+    child's counters (a synthetic capture; the real one runs on the GPU box)."""
+    bench = load_bench()
     hdr = '"ID","Process ID","Process Name","Host Name","Kernel Name","Context","Stream","Block Size","Grid Size","Device","CC","Section Name","Metric Name","Metric Unit","Metric Value"'
 
     def row(i, kernel, metric, unit, value):
